@@ -451,6 +451,59 @@ def run_c5(args):
         dist.destroy_process_group()
 
 
+DUMP_BYTE_SAMPLE = 1 << 21          # re-emitted byte positions in the dump (seeded, fixed for a given input size)
+DUMP_MAX_STREAMS = 4096             # streams whose verdicts, states and usage records are dumped (all of them at the default size)
+DUMP_MAX_BYTES = 64 << 20
+
+
+def _c3_outputs(eng, batch_set, dev) -> dict:
+    """What a caller of the device step holds after one step, as float arrays: the re-emitted bytes (a seeded sample of
+    positions), each stream's segment verdict, and each stream's state with the usage record the tap extracted."""
+    import torch
+    from llmapigateway_b200._abi import KIND_FLOAT, KIND_INT
+    from llmapigateway_b200.engine import SEG_DTYPE
+    b, h, d = batch_set
+    rng = np.random.default_rng(0)
+    n_bytes, n_streams = int(b.data.size), int(b.seg_slot.size)
+    pos = np.unique(rng.integers(0, n_bytes, size=min(n_bytes, DUMP_BYTE_SAMPLE)))
+    out = {"out_bytes_pos": pos.astype(np.float64),
+           "out_bytes": d["out"][torch.from_numpy(pos).to(dev)].cpu().numpy().astype(np.float32)}
+    sel = np.arange(n_streams) if n_streams <= DUMP_MAX_STREAMS else np.sort(rng.choice(n_streams, DUMP_MAX_STREAMS, replace=False))
+    out["stream_index"] = sel.astype(np.float64)
+    segs = d["segs"].cpu().numpy().view(SEG_DTYPE)[sel]
+    for f in SEG_DTYPE.names:
+        out["seg_" + f] = segs[f].astype(np.float64)
+    st = np.ctypeslib.as_array(eng.state(b.seg_slot[sel]))
+    for f in st.dtype.names:
+        if f != "rec":
+            out["state_" + f] = st[f].astype(np.float64)
+    rec = st["rec"]
+    for f in ("prompt_tokens", "completion_tokens", "total_tokens", "reasoning_tokens", "cached_tokens", "cost", "model_val", "provider_val"):
+        bits, kind = rec[f]["bits"], rec[f]["kind"]
+        val = np.zeros(len(sel))                    # 0 where the value is not a number (string, null, absent ...): `_kind` says which
+        val[kind == KIND_INT] = bits[kind == KIND_INT]
+        val[kind == KIND_FLOAT] = bits[kind == KIND_FLOAT].view(np.float64)
+        out["usage_" + f] = val
+        out["usage_" + f + "_kind"] = kind.astype(np.float64)
+    for f in ("model", "provider"):
+        raw = rec[f].view(np.uint8).reshape(len(sel), -1)
+        live = np.arange(raw.shape[1])[None, :] < rec[f + "_len"][:, None]       # bytes past the length are not part of the value
+        out["usage_" + f + "_bytes"] = np.where(live, raw, 0).astype(np.float32)
+        out["usage_" + f + "_len"] = rec[f + "_len"].astype(np.float64)
+    out["usage_str_flags"] = rec["str_flags"].astype(np.float64)
+    out["usage_exotic"] = rec["exotic"].astype(np.float64)
+    return out
+
+
+def _write_outputs(path: str, arrays: dict) -> None:
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, f"dump of {total} bytes exceeds {DUMP_MAX_BYTES}"
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64) and np.isfinite(a).all(), (name, a.dtype)
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def _emit(line: dict) -> None:
     data = (json.dumps(line) + "\n").encode()
     if _RESULT_FD is None:
@@ -473,7 +526,15 @@ def main():
                     help="c3 (default): BASELINE configs[2], the headline; c4: 3-deep fallback chain with 20 %% injected failure, 8192 streams "
                          "sharded over the GPUs (strong scaling); c5: usage rollup of 10 M records, 1 vs N GPUs")
     ap.add_argument("--records", type=int, default=10_000_000)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="c3: write what the last timed step computed as DIR/<name>.npy (float32/float64, at most 64 MB in all; "
+                         "a seeded sample of the re-emitted bytes), so that two builds can be compared output for output; "
+                         "e.g. bench_outputs/<build> (git-ignored)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.config != "c3" or args.impl != "b200"):
+        ap.error("--dump-outputs is implemented for the default configuration (--config c3 --impl b200)")
     # stdout carries exactly one line, the JSON result: everything else that writes to fd 1 during the run (NCCL's
     # version banner, library chatter of child processes) is sent to stderr
     global _RESULT_FD
@@ -576,6 +637,7 @@ def main():
     barrier()
     t_wall = time.perf_counter() - t_wall0
     launches = eng.launch_count() - l0
+    outputs = _c3_outputs(eng, sets[(K - 1) % 2], dev) if args.dump_outputs and rank == 0 else None     # (before anything reuses the set)
     dev_ms = float(np.sum(step_ms))
     if world > 1:
         t = torch.tensor([dev_ms], device=dev); dist.all_reduce(t, op=dist.ReduceOp.MAX); dev_ms = float(t.item())
@@ -743,6 +805,8 @@ def main():
             eng2.close_engine()
         except Exception as ex:                                    # never lose the headline line to a side measurement
             line["other_rows"] = {"error": repr(ex)}
+    if outputs is not None:
+        _write_outputs(args.dump_outputs, outputs)
     _emit(line)
     if world > 1:
         dist.destroy_process_group()

@@ -1,6 +1,6 @@
 """The reference's OWN code as the CPU arm -- TEST INFRASTRUCTURE (bench.py's cpu_baseline / --impl reference legs only).
 
-Drives, unmodified, from oracle/_ref (a copy of /root/reference made by oracle/build_ref.py):
+Drives, unmodified, from oracle/_ref (a copy of the reference made by oracle/build_ref.py):
   llm_gateway_core/services/request_handler.py:8     make_llm_request(..., is_streaming=True)  -- stream_generator,
         priming loop, combined_generator (loop A) over an httpx.MockTransport upstream (no sockets)
   llm_gateway_core/middleware/chat_logging.py:69     ChunkProcessorThread.run (loop B) + get_token_usage :233 on the
@@ -26,14 +26,11 @@ import types
 from pathlib import Path
 
 HERE = Path(__file__).resolve().parent
-REF_DIRS = [HERE / "_ref", Path("/root/reference")]
+REF_DIR = HERE / "_ref"
 
 
 def ref_root() -> Path | None:
-    for d in REF_DIRS:
-        if (d / "llm_gateway_core" / "services" / "request_handler.py").exists():
-            return d
-    return None
+    return REF_DIR if (REF_DIR / "llm_gateway_core" / "services" / "request_handler.py").exists() else None
 
 
 def _pure_python_loads():
@@ -67,12 +64,12 @@ _mods = {}
 
 
 def load(variant: str):
-    """Import the reference modules from oracle/_ref (or /root/reference) with the json5 stand-in of `variant`."""
+    """Import the reference modules from oracle/_ref with the json5 stand-in of `variant`."""
     if _mods.get("variant") == variant:
         return _mods["rh"], _mods["cl"]
     root = ref_root()
     if root is None:
-        raise RuntimeError("reference sources not available (oracle/_ref missing: run oracle/build_ref.py where /root/reference exists)")
+        raise RuntimeError("reference sources not available (oracle/_ref missing: run oracle/build_ref.py next to a reference checkout)")
     install_json5(variant)
     if str(root) not in sys.path:
         sys.path.insert(0, str(root))

@@ -45,7 +45,6 @@ def test_runs_once(engine):
 
 
 # ---- host half: write_log ---------------------------------------------------------------------------------------------------
-REF = Path("/root/reference")
 USAGE = {"prompt_tokens": 10, "completion_tokens": 5, "total_tokens": 17, "reasoning_tokens": 2, "cached_tokens": 4, "cost": 0.00123,
          "model": "m-ok", "provider": "P"}
 GOLDEN_LOG = Path(__file__).parent / "golden" / "write_log_cases.json"
