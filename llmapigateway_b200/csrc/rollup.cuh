@@ -7,8 +7,14 @@
 //
 // Every accumulator is an integer, so partial tables from several GPUs merge with a plain sum in
 // any order: token sums/count are int64; cost is summed EXACTLY as a 128-bit fixed-point number
-// (LSB 2^-80) held as four 32-bit limbs in 64-bit cells, then rounded once to double.  SQLite's
-// own SUM(REAL) is a compensated sum, so the two agree to an ulp or so (tests allow 4 ulp).
+// (LSB 2^-80) held as four 32-bit limbs in 64-bit cells, then rounded once to double (correctly
+// rounded, half to even: tests/test_rollup_cost_cpu.py pins it bit for bit against math.fsum).
+// A record is representable when it is finite, |c| < 2^15 and c * 2^80 is an integer; a group of
+// fewer than 2^32 such records cannot leave the 128-bit range (2^32 * 2^15 * 2^80 = 2^127), nor can a
+// 64-bit limb cell overflow.  A group holding any other record, or 2^32 records or more, is flagged
+// `inexact`; the host answers those groups from its own copy of the records, like SQLite
+// (usage.py: sqlite_sum).  SQLite's SUM(REAL) is a compensated sum, so unflagged groups agree
+// with it to an ulp or so (tests allow 4 ulp).
 //
 // Bucket index (monotone in time, so descending index == "time_period DESC"):
 //   hour  : day * 24 + hour-of-day          day : days since 1970-01-01   (day: see date_days)
@@ -87,7 +93,7 @@ LGW_RHD int64_t bucket_of(int64_t ts_us, int period) {
 
 // ---- exact cost accumulation ---------------------------------------------------------------------
 // double -> signed 128-bit fixed point with LSB 2^-80, as four 32-bit limbs (two's complement).
-// returns false when the value cannot be represented exactly (tiny bits lost, huge, NaN/Inf).
+// returns false when the value cannot be represented exactly (bits below 2^-80, |c| >= 2^15, NaN/Inf).
 LGW_RHD bool cost_to_limbs(double c, uint32_t limb[4]) {
     uint64_t b; memcpy(&b, &c, 8);
     const int E = (int)((b >> 52) & 0x7FF);
@@ -101,9 +107,8 @@ LGW_RHD bool cost_to_limbs(double c, uint32_t limb[4]) {
     bool exact = true;
     uint64_t lo, hi;
     if (shift >= 0) {
-        if (shift > 74) return false;                                 // |value| >= 2^47
-        if (shift >= 64) { lo = 0; hi = M << (shift - 64); }
-        else if (shift == 0) { lo = M; hi = 0; }
+        if (shift > 42) return false;                                 // |value| >= 2^15: 2^32 records could wrap the 128-bit sum
+        if (shift == 0) { lo = M; hi = 0; }
         else { lo = M << shift; hi = M >> (64 - shift); }
     } else {
         const int r = -shift;
@@ -348,7 +353,8 @@ __global__ void __launch_bounds__(1024) k_rollup_write(const unsigned long long*
     if (has && pos < rows_cap) {
         const unsigned long long* c = table + g * LGW_ROLLUP_CELLS;
         RollupRow r;
-        r.bucket = bucket0 + (int64_t)(g / n_models); r.model_rank = (int32_t)(g % n_models); r.inexact = inexact[g];
+        r.bucket = bucket0 + (int64_t)(g / n_models); r.model_rank = (int32_t)(g % n_models);
+        r.inexact = inexact[g] | (uint32_t)(c[5] >> 32 != 0);          // >= 2^32 records: the cost cells may have wrapped
         r.prompt_tokens = (int64_t)c[0]; r.completion_tokens = (int64_t)c[1]; r.total_tokens = (int64_t)c[2];
         r.reasoning_tokens = (int64_t)c[3]; r.cached_tokens = (int64_t)c[4]; r.count = (int64_t)c[5];
         uint64_t cells[4] = {c[6], c[7], c[8], c[9]};

@@ -8,10 +8,13 @@ llm_gateway_core/db/tokens_usage_db.py (TokensUsageDB) for rows a10/a11 of SURVE
 Records live as SoA columns (40 B/record) in HBM; `model` is dictionary-encoded at ingest and
 ranked in byte order so that ascending rank == the SQL's `model ASC`.  Every accumulator of the
 rollup is an integer (see csrc/rollup.cuh), so per-GPU partial tables merge with a plain sum.
+A group whose cost the fixed-point sum cannot hold (flag `inexact`) is answered on the host from
+the host copy of its records, the way SQLite sums them (`sqlite_sum`).
 """
 from __future__ import annotations
 
 import ctypes as C
+import math
 from datetime import datetime, timedelta
 
 import numpy as np
@@ -41,6 +44,43 @@ def period_label(period: str, bucket: int) -> str:
     if period == "week":
         return "%04d-W%02d" % (bucket // 64, bucket % 64)
     return "%04d-%02d" % (bucket // 12, bucket % 12 + 1)
+
+
+def sqlite_sum(costs) -> float | None:
+    """SUM(cost) of SQLite >= 3.43 over REAL values in scan order (Kahan-Babuska-Neumaier).  A NaN was stored as NULL and is
+    skipped; no value left gives NULL (None); a NaN result is NULL too.  A NaN error term is dropped, which is how [inf, 1.0]
+    sums to inf; an infinite one is not, so a sum that overflows, [1e308, 1e308], is inf + -inf = NULL."""
+    s = err = 0.0
+    seen = False
+    for r in costs:
+        if r != r:
+            continue
+        seen = True
+        t = s + r
+        err += (s - t) + r if abs(s) > abs(r) else (r - t) + s
+        s = t
+    if not seen:
+        return None
+    out = s if math.isnan(err) else s + err
+    return None if math.isnan(out) else out
+
+
+def _bucket_span_us(period: str, bucket: int) -> tuple[int, int]:
+    """[lo, hi) in microseconds holding every timestamp whose bucket_of() is `bucket`, with the one-day slack of SQLite's
+    millisecond roll (csrc/rollup.cuh: a record can land in the bucket of the next day)."""
+    day = 86400 * 10**6
+    if period == "hour":
+        return (bucket - 24) * 3600 * 10**6, (bucket + 1) * 3600 * 10**6
+    if period == "day":
+        return (bucket - 1) * day, (bucket + 1) * day
+    if period == "month":
+        y, m = divmod(bucket, 12)
+        first = to_us(datetime(y, m + 1, 1))
+        nxt = to_us(datetime(y + 1, 1, 1) if m == 11 else datetime(y, m + 2, 1))
+        return first - day, nxt
+    y, w = divmod(bucket, 64)                 # %W = (day of year + 7 - weekday) / 7: day of year in [7w - 7, 7w + 5]
+    jan1 = to_us(datetime(y, 1, 1))
+    return jan1 + (7 * w - 8) * day, jan1 + (7 * w + 6) * day
 
 
 def stats_window(period: str, now: datetime):
@@ -205,11 +245,21 @@ class UsageTable:
                                                      rows.ctypes.data_as(C.c_void_p), groups, C.byref(n_rows)), "usage_rollup_emit")
         return rows[:n_rows.value]
 
+    def _row_dict(self, period: str, r, cost) -> dict:
+        return {"time_period": period_label(period, int(r["bucket"])), "model": self._names[int(r["model_rank"])],
+                "prompt_tokens": int(r["prompt_tokens"]), "completion_tokens": int(r["completion_tokens"]),
+                "total_tokens": int(r["total_tokens"]), "reasoning_tokens": int(r["reasoning_tokens"]),
+                "cached_tokens": int(r["cached_tokens"]), "cost": cost, "count": int(r["count"])}
+
     def rows_to_dicts(self, period: str, rows) -> list[dict]:
-        return [{"time_period": period_label(period, int(r["bucket"])), "model": self._names[int(r["model_rank"])],
-                 "prompt_tokens": int(r["prompt_tokens"]), "completion_tokens": int(r["completion_tokens"]),
-                 "total_tokens": int(r["total_tokens"]), "reasoning_tokens": int(r["reasoning_tokens"]),
-                 "cached_tokens": int(r["cached_tokens"]), "cost": float(r["cost"]), "count": int(r["count"])} for r in rows]
+        """Dicts of emitted rows (e.g. of a table all-reduced over ranks).  A row flagged `inexact` is refused with ValueError:
+        its cost is not the sum of its records, and the records that would give the right answer may live on other ranks."""
+        bad = np.flatnonzero(rows["inexact"])
+        if bad.size:
+            r = rows[bad[0]]
+            raise ValueError("%d rollup row(s) hold a cost the fixed-point sum cannot represent (first: %s, model %r)"
+                             % (bad.size, period_label(period, int(r["bucket"])), self._names[int(r["model_rank"])]))
+        return [self._row_dict(period, r, float(r["cost"])) for r in rows]
 
     def rollup_rows(self, period: str, start: datetime | None = None, end: datetime | None = None) -> np.ndarray:
         """Rows (ROW_DTYPE) ordered time_period DESC, model ASC."""
@@ -242,13 +292,25 @@ class UsageTable:
         if len(self) == 0:
             return []
         rows = self.rollup_rows(period, start_date, end_date)
-        out = []
-        for r in rows:
-            out.append({"time_period": period_label(period, int(r["bucket"])), "model": self._names[int(r["model_rank"])],
-                        "prompt_tokens": int(r["prompt_tokens"]), "completion_tokens": int(r["completion_tokens"]),
-                        "total_tokens": int(r["total_tokens"]), "reasoning_tokens": int(r["reasoning_tokens"]),
-                        "cached_tokens": int(r["cached_tokens"]), "cost": float(r["cost"]), "count": int(r["count"])})
-        return out
+        cost = rows["cost"].tolist()
+        for j in np.flatnonzero(rows["inexact"]).tolist():
+            cost[j] = sqlite_sum(self._group_costs(period, start_date, end_date, int(rows["bucket"][j]), int(rows["model_rank"][j])))
+        return [self._row_dict(period, r, c) for r, c in zip(rows, cost)]
+
+    def _group_costs(self, period: str, start: datetime | None, end: datetime | None, bucket: int, model_rank: int) -> list[float]:
+        """Costs of one group's records from the host columns, in insertion order (SQLite's scan order within a group).
+        numpy narrows the records to the model and a time span around the bucket; bucket_of() decides the rest."""
+        h = self._host
+        ts = h["ts_us"]
+        lo, hi = _bucket_span_us(period, bucket)
+        sel = (h["model_rank"] == model_rank) & (ts >= lo) & (ts < hi)
+        if start is not None:
+            sel &= ts >= to_us(start)
+        if end is not None:
+            sel &= ts <= to_us(end)
+        p = PERIODS[period]
+        keep = [i for i in np.flatnonzero(sel).tolist() if self._lib.lgw_rollup_bucket_of(int(ts[i]), p) == bucket]
+        return h["cost"][keep].tolist()
 
     # -- record listing: /v1/api/usage-records (stats.py:69-87) ---------------------------------------------
     def get_total_records_count(self) -> int:

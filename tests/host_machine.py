@@ -157,3 +157,25 @@ def doc_usage(raw: bytes):
     buf = np.frombuffer(raw, dtype=np.uint8) if raw else np.zeros(1, np.uint8)
     lib().lgwt_doc_usage(buf.ctypes.data_as(C.c_void_p), C.c_uint32(len(raw)), C.byref(out))
     return out
+
+
+def cost_to_limbs(c: float):
+    """rollup.cuh cost_to_limbs(): (exact, the four 32-bit limbs of c * 2^80, two's complement, low limb first)"""
+    limb = (C.c_uint32 * 4)()
+    ok = lib().lgwt_cost_to_limbs(C.c_double(c), limb)
+    return bool(ok), tuple(limb)
+
+
+def limbs_to_cost(cells) -> float:
+    """rollup.cuh limbs_to_cost() of four 64-bit cells (Python ints, taken mod 2^64)"""
+    f = lib().lgwt_limbs_to_cost
+    f.restype = C.c_double
+    return f((C.c_uint64 * 4)(*[int(x) % 2**64 for x in cells]))
+
+
+def sum_costs(costs) -> tuple[bool, tuple]:
+    """the limbs of every cost summed into four 64-bit cells as the kernels do: (all exact, cells)"""
+    a = np.ascontiguousarray(costs, np.float64)
+    cell = (C.c_uint64 * 4)()
+    ok = lib().lgwt_sum_costs(a.ctypes.data_as(C.c_void_p), C.c_uint64(a.size), cell)
+    return bool(ok), tuple(cell)

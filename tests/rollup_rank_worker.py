@@ -29,6 +29,8 @@ def main():
     n = 200_000
     ts, models, tok, cost = U.synth_usage_columns(n, seed=11, end=NOW)
     names = sorted({m for m in models if m is not None})
+    flagged = n - 1                                         # one record of rank 1's half the fixed-point cost sum cannot hold
+    ts[flagged], models[flagged], cost[flagged] = U.to_us(NOW - timedelta(days=1)), names[0], float("inf")
     if rank == 1:
         names_local_missing = names[-1]                     # rank 1 never sees the rarest model: the shared dictionary must still line up
         keep = np.array([m != names_local_missing for m in models])
@@ -62,7 +64,18 @@ def main():
             from test_rollup_gpu import _compare, _iso
             rows = tab.emit(b0, nb, nm, C.c_void_p(table.data_ptr()), C.c_void_p(inexact.data_ptr()))
             conn = ro.make_db([(_iso(ts[i]), int(tok[0][i]), int(tok[1][i]), int(tok[2][i]), int(tok[3][i]), int(tok[4][i]), float(cost[i]), models[i], "P") for i in range(n)])
-            _compare(tab.rows_to_dicts(period, rows), ro.aggregated_usage(conn, period, start, end))
+            want = ro.aggregated_usage(conn, period, start, end)
+            # the merged row of the flagged record's group carries the flag, and rows_to_dicts refuses to print its cost
+            key = (U.period_label(period, int(tab._lib.lgw_rollup_bucket_of(int(ts[flagged]), p))), names[0])
+            bad = np.flatnonzero(rows["inexact"])
+            assert [(U.period_label(period, int(rows["bucket"][j])), tab._names[int(rows["model_rank"][j])]) for j in bad] == [key], (period, bad)
+            try:
+                tab.rows_to_dicts(period, rows)
+                raise AssertionError("rows_to_dicts printed a flagged row")
+            except ValueError:
+                pass
+            assert [w["cost"] for w in want if (w["time_period"], w["model"]) == key] == [float("inf")]
+            _compare(tab.rows_to_dicts(period, np.delete(rows, bad)), [w for w in want if (w["time_period"], w["model"]) != key])
     dist.barrier()
     dist.destroy_process_group()
     if rank == 0:

@@ -1,4 +1,4 @@
-// TEST AID ONLY: compiles the device-side machines (json_machine.cuh / stream_machine.cuh) for
+// TEST AID ONLY: compiles the device-side machines (json_machine.cuh / stream_machine.cuh, rollup.cuh) for
 // the host so the CPU test-suite can fuzz them against CPython and the oracle without a GPU.
 // Never linked into the product library; the product has no CPU path.
 #include <stddef.h>
@@ -136,4 +136,20 @@ extern "C" void lgwt_doc_usage(const uint8_t* doc, uint32_t len, lgw_doc_usage* 
             if (f & TK_ERROR) out->error_row = 1;                        // :137-139
         }
     }
+}
+
+// ---- exact cost accumulation of the usage rollup (rollup.cuh): the same integer code the kernels run ---------------------
+#include "../../llmapigateway_b200/csrc/rollup.cuh"
+extern "C" int lgwt_cost_to_limbs(double c, uint32_t limb[4]) { return lgw::cost_to_limbs(c, limb) ? 1 : 0; }
+extern "C" double lgwt_limbs_to_cost(const uint64_t cell[4]) { return lgw::limbs_to_cost(cell); }
+// the limbs of n records added into four 64-bit cells (wrap-around) as the rollup kernels add them; 0 when any record was not exact
+extern "C" int lgwt_sum_costs(const double* c, uint64_t n, uint64_t cell[4]) {
+    int exact = 1;
+    cell[0] = cell[1] = cell[2] = cell[3] = 0;
+    for (uint64_t i = 0; i < n; ++i) {
+        uint32_t limb[4];
+        exact &= lgw::cost_to_limbs(c[i], limb) ? 1 : 0;
+        for (int k = 0; k < 4; ++k) cell[k] += limb[k];
+    }
+    return exact;
 }
